@@ -18,9 +18,11 @@ Prints ONE JSON line (rank 0).  `value`   : device-timed (CUDA events) images/s,
                                             calls on host arrays, 8 caller threads; the one-thread number, the
                                             standalone-NMS numbers and the build's streaming API are reported beside it.
                                 `roofline`: the conv/GEMM tensor-core kernel, timed live per launch (frac vs the burst
-                                            peak), a >= 200-image sustained run (vs the sustained peak), DRAM traffic and
+                                            peak), a second run of the lanes (vs the sustained peak), DRAM traffic and
                                             per-kernel HBM fractions from the committed ncu pass of this binary.
                                 `cpu_baseline`: the CPU oracle pipeline on this box's host cores (rank 0, N=1).
+Every timed leg of the B200 arm runs --steps images.  `--dump-outputs DIR` writes what the last timed image computed
+(see dump_outputs); the inputs are seeded, so two builds can be compared output for output.
 `--impl reference` times the reference-equivalent CPU pipeline instead (torch-CPU fp32 dense ops standing in for
 Chainer-NumPy -- Chainer is not installable offline -- plus the reference's own compiled cpu_nms.pyx when
 oracle/_ref holds it, else the C restatement).
@@ -347,6 +349,19 @@ def reference_api_image(model, x_var, info_var, nms, np_):
     return prob.shape[0], n_det
 
 
+def dump_outputs(out_dir, plan):
+    """Writes what the caller of the timed path receives for the image `plan` ran last: the proposals (rois, scores), the
+    class probabilities (prob), the decoded boxes (boxes) and the per-class NMS result (keep_idx per class with entries
+    past keep_count set to -1, keep_count, conf_count) as out_dir/<name>.npy.  Integers are stored as float64 (exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    r = plan.unpack_result(plan.result.cpu().numpy())
+    r["count"] = np.array([r["count"]])
+    r["keep_idx"] = np.where(np.arange(r["keep_idx"].shape[1]) < r["keep_count"][:, None], r["keep_idx"], -1)
+    for name, a in r.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 def run_b200_arm(args, rank, local_rank, world):
     import torch
     import frcnn_oracle as orc              # synthetic weights / image generators + cpu_baseline only
@@ -400,11 +415,13 @@ def run_b200_arm(args, rank, local_rank, world):
     e0.record()
     pool.fork()
     for i in range(args.steps):
-        pool.submit(i, imgs_dev[i % n_img])          # every step = one whole image through the whole path
+        last = pool.submit(i, imgs_dev[i % n_img])   # every step = one whole image through the whole path
     pool.join()
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)        # before the legs below reuse the lanes' buffers
     R_last = int(plan.prop.count.item())
     n_conf_last = int(plan.det[2].sum().item())
     # tie-free-ness of the run (SURVEY 8d): distinct fg scores among the anchors of the last image
@@ -418,8 +435,9 @@ def run_b200_arm(args, rank, local_rank, world):
     e1.record()
     barrier()
     ms_single = e0.elapsed_time(e1)
-    # a sustained run (>= 200 images, whatever --steps says): the number to hold against bf16_tflops_sustained
-    n_sus = max(200, args.steps)
+    # the lanes once more after the legs above: the number to hold against bf16_tflops_sustained (a long --steps makes it
+    # a sustained run; every timed leg runs --steps images)
+    n_sus = args.steps
     barrier()
     e0.record()
     pool.fork()
@@ -434,7 +452,7 @@ def run_b200_arm(args, rank, local_rank, world):
     table = conv_layer_table(plan, torch) if rank == 0 else None
     ms_max = shard.max_over_ranks(ms, device="cuda")          # slowest rank decides
     value = world * args.steps / (ms_max / 1e3)
-    # seeds 0-4 (SURVEY 8d): one image in flight, 20 images per seed, this rank
+    # seeds 0-4 (SURVEY 8d): one image in flight, --steps images per seed, this rank
     seed_rates = {}
     if rank == 0:
         for sd in range(5):
@@ -442,11 +460,11 @@ def run_b200_arm(args, rank, local_rank, world):
             plan.forward(xi)
             torch.cuda.synchronize()
             e0.record()
-            for _ in range(20):
+            for _ in range(args.steps):
                 plan.forward(xi)
             e1.record()
             torch.cuda.synchronize()
-            seed_rates[str(sd)] = {"images_per_s": 20e3 / e0.elapsed_time(e1), "proposals": int(plan.prop.count.item())}
+            seed_rates[str(sd)] = {"images_per_s": args.steps * 1e3 / e0.elapsed_time(e1), "proposals": int(plan.prop.count.item())}
     barrier()
 
     # The e2e legs run Python per image.  A full (generation-2) garbage collection in a process that has imported torch walks
@@ -560,8 +578,7 @@ def run_b200_arm(args, rank, local_rank, world):
     import sys as _sys
     old_switch = _sys.getswitchinterval()
     _sys.setswitchinterval(1e-4)
-    n_thr = max(args.steps, 6 * T)           # at least 6 images per caller thread, whatever --steps says (reported: e2e.images_timed)
-    per = [(n_thr + T - 1 - k) // T for k in range(T)]
+    per = [(args.steps + T - 1 - k) // T for k in range(T)]          # --steps images over the T threads (e2e.images_timed)
 
     def threads_leg():
         errs = []
@@ -958,6 +975,8 @@ def main():
     ap.add_argument("--smem-reserve-kb", type=int, default=0,
                     help="shared memory per SM the conv kernels leave to other streams' small kernels (tuning experiment)")
     ap.add_argument("--api-threads", type=int, default=8, help="caller threads of the reference-interface e2e leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="forward workload: write the results of the last timed image as DIR/<name>.npy (rank 0)")
     ap.add_argument("--workload", default="forward", choices=["forward", "train_rpn", "train_rcnn", "resnet101"],
                     help="forward = the headline metric (default); train_rpn / resnet101 = secondary workloads (configs #5 / #4)")
     args = ap.parse_args()

@@ -91,6 +91,16 @@ def import_reference():
     return Variable, ref_nms, ga, bt, pl
 
 
+def write_cpu_nms_clustered(ref_nms):
+    """cpu_nms keep lists on larger clustered cases (1500 boxes, 40 clusters) at the three thresholds the project uses."""
+    out = {}
+    for name, (seed, thr) in gi.NMS_CLUSTERED_CASES.items():
+        dets = gi._clustered_dets(1500, seed)
+        out[name + "_keep"] = np.asarray(ref_nms.cpu_nms(dets, thr), dtype=np.int64)
+        out[name + "_checksum"] = gi.checksum(dets)
+    np.savez_compressed(os.path.join(HERE, "cpu_nms_clustered.npz"), **out)
+
+
 def main():
     Variable, ref_nms, ga, bt, pl = import_reference()
     out = {}
@@ -124,6 +134,7 @@ def main():
         out[name + "_thr"] = np.float64(thr)
         out[name + "_checksum"] = gi.checksum(dets)
     np.savez(os.path.join(HERE, "cpu_nms.npz"), **out)
+    write_cpu_nms_clustered(ref_nms)
 
     # ---- 4. ProposalLayer.__call__
     out = {}

@@ -79,6 +79,11 @@ NMS_CASES = {
 }
 
 
+# name: (seed of _clustered_dets(1500, seed), threshold)
+NMS_CLUSTERED_CASES = {"s%d_t%02d" % (seed, round(10 * thr)): (seed, thr)
+                       for seed in range(100, 105) for thr in (0.3, 0.5, 0.7)}
+
+
 def nms_case(name):
     n, thr = NMS_CASES[name]
     seed = zlib.crc32(name.encode()) & 0xFFFF

@@ -6,7 +6,7 @@
     probability errors PER ELEMENT (not only max-norm), printed and asserted;
   * the reference's interface: models.faster_rcnn.FasterRCNN.__call__ fed HOST float32 arrays (one pinned upload, one
     download) returns bit for bit what the device path returns, also from several caller threads at once;
-  * the reference's own test files executed unchanged (when /root/reference is present -- it is not on the GPU box);
+  * the calls of the reference's own tests, compared with the outputs the reference returned (tests/golden);
   * the training path's NCCL all-reduce as a pytest (skipped under 2 GPUs).
 
 Tolerance readings ("within 1e-4 relative", BASELINE north_star):
@@ -354,45 +354,40 @@ def test_cpu_nms_host_small_and_large_paths_and_threads():
     assert not errs, errs
 
 
-# ------------------------------------------------------------------------------- the reference's own test files, unchanged
-REF = "/root/reference"
-
-
-def _run_reference_test_file(rel, only=None):
-    """Load /root/reference/<rel> as a module (unchanged source) after dropin.install() and run its unittest cases."""
-    import importlib.util
-    import unittest
+# ------------------------------------------------------------------------------- the reference's own test calls vs its outputs
+@pytest.mark.parametrize("case", ["generate_anchors_s4-32", "generate_anchors_s8-32", "proposal_layer_cpu", "proposal_layer_gpu"])
+def test_reference_test_calls_vs_reference_golden(golden_dir, case):
+    """The calls of the reference's tests/test_generate_anchors.py and tests/test_proposal_layer.py, made on this build's
+    `models` package (dropin.install()) and compared with what the reference itself returned for the same inputs
+    (tests/golden/anchors.npz, proposal_layer.npz case t14_train: a 14x14 map, img_info 224x224, train-mode top-n).
+    The statements of its RegionProposalNetwork and FasterRCNN tests are re-typed in test_dropin_gpu.py and below."""
+    import chainer
+    from chainer import Variable
     from frcnn_b200 import dropin
+    import golden_inputs as gi
     dropin.install()
-    path = os.path.join(REF, rel)
-    name = "ref_" + os.path.basename(rel)[:-3]
-    spec = importlib.util.spec_from_file_location(name, path)
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules[name] = mod
-    spec.loader.exec_module(mod)
-    suite = unittest.defaultTestLoader.loadTestsFromModule(mod)
-
-    def flatten(s):
-        for t in s:
-            if isinstance(t, unittest.TestSuite):
-                for u in flatten(t):
-                    yield u
-            else:
-                yield t
-    tests = [t for t in flatten(suite) if only is None or only in t.id()]
-    assert tests, "no test cases found in %s" % rel
-    res = unittest.TextTestRunner(verbosity=0).run(unittest.TestSuite(tests))
-    assert res.wasSuccessful(), (res.failures, res.errors)
-    return len(tests)
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference is not present on this box (it never is on the GPU box)")
-@pytest.mark.parametrize("rel,only", [("tests/test_proposal_layer.py", None), ("tests/test_region_proposal_network.py", None),
-                                      ("tests/test_generate_anchors.py", None), ("tests/test_faster_rcnn.py", "test_forward_whole")])
-def test_reference_test_files_run_unchanged(rel, only):
-    """The reference's own tests executed as files against this build's `models` package (dropin.install()); test_faster_rcnn.py
-    needs datasets.pascal_voc_dataset.VOC -> the synthetic stand-in in chainer-faster-rcnn_b200/datasets/."""
-    assert _run_reference_test_file(rel, only) > 0
+    if case.startswith("generate_anchors"):
+        from models.generate_anchors import generate_anchors
+        g = np.load(os.path.join(golden_dir, "anchors.npz"))
+        scales, key = {"s4-32": ((4, 8, 16, 32), "anchors_default_call"), "s8-32": ((8, 16, 32), "anchors_proposal_layer")}[case.split("_")[-1]]
+        assert np.array_equal(generate_anchors(15, (0.5, 1, 2), scales), g[key])
+        return
+    from models.proposal_layer import ProposalLayer
+    g = np.load(os.path.join(golden_dir, "proposal_layer.npz"))
+    prob, pred, info, train = gi.proposal_case("t14_train")
+    assert train and gi.checksum(prob, pred) == g["t14_train_checksum"]
+    layer = ProposalLayer()
+    if case == "proposal_layer_cpu":
+        rois, probs = layer(Variable(prob), Variable(pred), Variable(info))
+        assert isinstance(rois, np.ndarray) and isinstance(probs, np.ndarray)
+    else:
+        cp = chainer.cuda.cupy
+        rois, probs = layer(Variable(cp.asarray(prob)), Variable(cp.asarray(pred)), Variable(info.astype(np.int64)))
+        assert isinstance(rois, cp.ndarray)
+        rois, probs = cp.asnumpy(rois), cp.asnumpy(probs)
+    assert rois.shape == g["t14_train_rois"].shape and probs.shape == g["t14_train_probs"].shape
+    assert np.array_equal(probs, g["t14_train_probs"])                   # scores are copied, never recomputed: exact
+    np.testing.assert_allclose(rois, g["t14_train_rois"], rtol=2e-6, atol=1e-3)     # numpy's exp vs the pinned one
 
 
 def test_reference_test_faster_rcnn_statements_with_the_voc_stand_in():
